@@ -197,6 +197,7 @@ def run_ours(a):
     e1.record()
     barrier()
     launches = L.LAUNCHES - launches0
+    dumped = {"page_reps": reps.float().cpu().numpy()} if a.dump_outputs else None
     clocks = sampler.stop() if rank == 0 else None
     ms_total = max_over_ranks(e0.elapsed_time(e1))
     value = world * a.steps * P / (ms_total / 1e3)
@@ -222,6 +223,8 @@ def run_ours(a):
     intervals = [round((b - a_) * 1e3, 1) for a_, b in zip(marks, marks[1:])]  # first one includes the pipeline fill
     e2e_value = world * a.steps * P / (e2e_ms / 1e3)
     host_reps = torch.from_numpy(host_np)
+    if dumped is not None:
+        dumped["e2e_page_reps"] = host_np.astype(np.float32)
     e0.record()
     for _ in range(a.steps):
         model(passage=items, tokenizer=tok, max_inp_length=2048).p_reps.cpu()
@@ -303,6 +306,9 @@ def run_ours(a):
     e1.record()
     barrier()
     q_ms = max_over_ranks(e0.elapsed_time(e1)) / a.query_reps
+    if dumped is not None:
+        dumped.update(query_reps=qe_all.float().cpu().numpy(), query_top10_scores=s_top.float().numpy(),
+                      query_top10_ids=i_top.numpy().astype(np.float64))  # ids are exact in float64
     qe = torch.nn.functional.normalize(torch.randn(nq, cfg.hidden, device=dev, generator=torch.Generator(device=dev).manual_seed(77)), dim=1)
     retriever.sharded_topk(qe, index, 10, lo)
     barrier()
@@ -480,8 +486,30 @@ def run_ours(a):
             "cpu_baseline": cpu_baseline, "torch_gpu_baseline": torch_arm, "setup_s": round(setup_s, 1),
         }
         print(json.dumps(line), flush=True)
+        if dumped is not None:
+            dump_outputs(a.dump_outputs, dumped)
     if world > 1:
         dist.destroy_process_group()
+
+
+def dump_outputs(out_dir, arrays):
+    """Writes what the timed paths returned in their last step as out_dir/<name>.npy (rank 0's share when N > 1):
+    page_reps       [pages, 2304] embeddings of the device-resident step (`value`)
+    e2e_page_reps   [pages, 2304] embeddings the host received from the last step of the e2e loop
+    query_reps      [queries, 2304] encoded text queries, query_top10_scores / _ids [queries, 10] their top-10.
+    All inputs are seeded, so runs with the same arguments compare output for output. Above 64 MB in all, every array
+    keeps the same fraction of its rows, chosen with a fixed seed (the same rows in every run with these arguments)."""
+    import numpy as np
+
+    limit = 64 << 20
+    total = sum(x.nbytes for x in arrays.values())
+    os.makedirs(out_dir, exist_ok=True)
+    for name, x in arrays.items():
+        assert x.dtype in (np.float32, np.float64), (name, x.dtype)
+        if total > limit:
+            keep = max(1, len(x) * limit // total)
+            x = x[np.sort(np.random.RandomState(0).choice(len(x), keep, replace=False))]
+        np.save(os.path.join(out_dir, f"{name}.npy"), x)
 
 
 def cpu_port_baseline(cfg, sd_cpu, tok, pages, page_px):
@@ -619,7 +647,11 @@ def main():
     ap.add_argument("--no-cpu-baseline", dest="cpu_baseline", action="store_false")
     ap.add_argument("--no-torch-baseline", dest="torch_baseline", action="store_false",
                     help="skip the stock-PyTorch-on-this-GPU context arm (N = 1 only)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the outputs of their last step to DIR/<name>.npy (see dump_outputs)")
     a = ap.parse_args()
+    if a.dump_outputs and a.impl != "ours":
+        ap.error("--dump-outputs is only implemented for --impl ours")
     if a.warmup < 3 and a.impl == "ours":
         a.warmup = 3
     if a.big_corpus < 0:

@@ -7,8 +7,8 @@ point, so it is plain fp32 PyTorch-on-CPU / numpy (third-party primitives the re
 ``F.interpolate``, ``F.layer_norm``, ``erf``-GELU, ``softmax``, ``PIL.Image.resize``).
 
 Pinning: the reference has NO tests or golden vectors for this path (SURVEY.md §4, F11). This oracle is
-pinned against the reference *itself*, executed in the build container through ``oracle/reference_shim.py``
-(``tests/test_oracle_vs_reference.py``, skipped when /root/reference is absent) and against the golden
+pinned against the reference *itself*, executed through ``oracle/reference_shim.py`` to produce
+``tests/golden/reference_checks.npz`` (``tests/test_oracle_vs_reference.py``) and against the golden
 vectors generated from the real reference by ``oracle/gen_golden.py`` (``tests/golden/*.npz``,
 ``tests/test_oracle_golden.py`` — runs everywhere).
 

@@ -1,132 +1,62 @@
-"""The drop-in classes under the REAL reference driver (build container only: needs /root/reference).
+"""The drop-in classes on the path the REAL reference driver takes, against what that driver produced.
 
-`src/openmatch/driver/eval.py` is imported unmodified; only the two names INTEGRATION.md §2.3 tells a maintainer to rebind are
-rebound: `DRModelForInference` (-> visrag_b200.modeling) and, for metrics, the absent `pytrec_eval` package (-> a shim over
-visrag_b200.inference's restated measures). Then the driver's own functions run:
-  setup_model (eval.py:118-134)  -> OUR DRModelForInference.build -> from_pretrained -> config.json + *.safetensors of a
-                                    synthetic HF checkpoint directory written by weights.save_checkpoint
-  the reference's distributed_parallel_embedding_inference (inference.py:53-172) drives the returned model with its own
-                                    DataLoader / naive_collator / kwargs conventions and writes the pickle shards
-  retrieve (eval.py:210-232)     -> the reference's CPU retrieval over those shards, save_as_trec, save_results
-There is no GPU in the build container, so the ONE thing replaced by test infrastructure is the device math: the model class
-under test is a subclass of visrag_b200's whose `encode` computes the embeddings with the oracle (CPU). Everything else -
-checkpoint discovery and loading, config translation, the B2 call conventions the driver relies on (.to/.eval/forward(query=,
-passage=, **kwargs) -> .q_reps/.p_reps tensors) - is the shipped code. The same `build()` runs on real kernels in
-tests/test_gpu_encode.py::test_build_from_checkpoint_directory."""
-import json
+tests/golden/driver_run.npz holds the outputs of the reference's `src/openmatch/driver/eval.py`, imported unmodified and
+driving this package's `DRModelForInference` on a synthetic checkpoint directory (oracle/gen_golden.py --checks):
+setup_model -> DRModelForInference.build, its distributed_parallel_embedding_inference (inference.py:53-172) writing
+the pickle shards, its retrieve phase (eval.py:210-232) writing the run file. Only the device math was replaced there
+(oracle embeddings on the CPU). Here the same checkpoint goes through the same calls of this package on the GPU:
+`build` (what setup_model calls, eval.py:118-134), `.to` / `.eval`, `inference.distributed_parallel_embedding_inference`
+and `retriever.distributed_parallel_retrieve` + `save_as_trec`; the shards and the run must be the reference driver's."""
 import os
-import sys
-import types
-from types import SimpleNamespace
 
 import numpy as np
 import pytest
-import torch
 
-from oracle import reference_shim as RS
-from tests.helpers import synth_doc_pages
+from tests.helpers import DRIVER_RUN, cosine_rows, driver_run_args, driver_run_inputs
 
-pytestmark = pytest.mark.skipif(not RS.available(), reason="needs /root/reference (build container only)")
+pytestmark = pytest.mark.gpu
 
 
-def _pytrec_eval_shim():
-    """pytrec_eval's two entry points used by eval.py:281-299, over visrag_b200.inference's restated measures."""
+def test_reference_driver_drives_the_dropin_classes(tmp_path):
+    from types import SimpleNamespace
+
     from visrag_b200 import inference as I
-
-    m = types.ModuleType("pytrec_eval")
-
-    class RelevanceEvaluator:
-        def __init__(self, qrels, measures):
-            self.qrels, self.measures = qrels, set(measures)
-
-        def evaluate(self, run):
-            rec, ndcg = I.recall_at_k(self.qrels, run, 10), I.ndcg_at_k(self.qrels, run, 10)
-            return {qid: {"recall_10": rec[qid], "ndcg_cut_10": ndcg[qid]} for qid in rec if qid != "all"}
-
-    m.RelevanceEvaluator = RelevanceEvaluator
-    m.compute_aggregated_measure = lambda measure, values: float(np.mean(values)) if values else 0.0
-    return m
-
-
-def test_reference_driver_drives_the_dropin_classes(tmp_path, monkeypatch):
-    from oracle import restated as O
-    from visrag_b200 import modeling as M
-    from visrag_b200.config import VisRAGConfig
+    from visrag_b200 import retriever as R
+    from visrag_b200.modeling import DRModelForInference
     from visrag_b200.tokenizer_stub import StubTokenizer
     from visrag_b200.weights import random_state_dict, save_checkpoint
 
-    R = RS._import_reference()
-    monkeypatch.setitem(sys.modules, "pytrec_eval", _pytrec_eval_shim())
-    import openmatch.driver.eval as ev
-    from openmatch.inference import distributed_parallel_embedding_inference as ref_inference
-
-    # ---- a synthetic checkpoint directory in the public checkpoint's layout
-    cfg = VisRAGConfig.tiny()
-    sd = random_state_dict(cfg, 77)
+    ref = np.load(DRIVER_RUN, allow_pickle=False)
+    cfg, seed, corpus, queries = driver_run_inputs()
     ckpt = str(tmp_path / "VisRAG-Ret-synthetic")
-    save_checkpoint(ckpt, cfg, sd)
-    assert ev.get_model_name(SimpleNamespace(model_name_or_path=ckpt)) == "VisRAG-Ret-synthetic"  # eval.py:306-316 reads our config.json
+    save_checkpoint(ckpt, cfg, random_state_dict(cfg, seed))
+    margs = SimpleNamespace(model_name_or_path=ckpt, pooling="wmean", normalize=True, cache_dir=None)
+    model = DRModelForInference.build(model_args=margs, cache_dir=margs.cache_dir)
+    assert model.to("cuda:0") is model and model.eval() is model
+    assert model.pooling == "wmean" and model.normalize is True and model.lm_q.config == cfg
 
-    # ---- the class under test: shipped build()/from_pretrained()/load_checkpoint(); device math -> oracle (no GPU here)
-    loaded = {}
+    args = driver_run_args(str(tmp_path / "out"), "cuda:0")
+    kw = {"tokenizer": StubTokenizer(cfg.vocab), "max_inp_length": 2048}
+    I.distributed_parallel_embedding_inference(corpus, model, args, dataset_type="corpus", split_save=True, model_additional_args=kw)
+    I.distributed_parallel_embedding_inference(queries, model, args, dataset_type="query", split_save=False, model_additional_args=kw)
+    names = sorted(f for f in os.listdir(args.output_dir) if f.startswith("embeddings."))
+    assert names == [str(n) for n in ref["shard_names"]]  # flush rule of inference.py:112 at max_inmem_docs=6
+    for n in names:
+        emb, ids = R.load_shard(os.path.join(args.output_dir, n))
+        assert ids == [str(i) for i in ref[f"{n}:ids"]], n
+        assert cosine_rows(emb, ref[f"{n}:reps"]).min() >= 0.9999, n
 
-    class HostBackbone(M.VisRAGRetB200):
-        def __init__(self, cfg_, state_dict, device="cuda:0"):
-            self.config, self.device, self.dtype, self.training = cfg_, torch.device("cpu"), torch.bfloat16, False
-            loaded["cfg"], loaded["sd"] = cfg_, {k: v.float() for k, v in state_dict.items()}
-
-    class HostDR(M.DRModelForInference):
-        def encode(self, items, model, head, is_query=False, **kwargs):
-            if items is None:
-                return None, None
-            assert self.normalize is True
-            reps = O.encode(loaded["sd"], loaded["cfg"], kwargs["tokenizer"], items["text"], items["image"],
-                            pooling=self.pooling, max_inp_length=kwargs.get("max_inp_length", 2048))
-            return None, torch.from_numpy(reps)
-
-    monkeypatch.setattr(M, "VisRAGRetB200", HostBackbone)   # build() instantiates the backbone class by this name
-    monkeypatch.setattr(ev, "DRModelForInference", HostDR)
-    model_args = R["ModelArguments"](model_name_or_path=ckpt, pooling="wmean", normalize=True)
-    out_dir = str(tmp_path / "out")
-    enc_args = SimpleNamespace(phase="encode", device="cpu", output_dir=out_dir, per_device_eval_batch_size=3, dataloader_num_workers=0,
-                               dataloader_pin_memory=False, fp16=False, max_inmem_docs=6, world_size=1, process_index=0,
-                               retrieve_depth=4, trec_save_path=None)  # the reference's torch.topk needs depth <= smallest shard
-    model = ev.setup_model(enc_args, model_args)                      # eval.py:118-134, unmodified
-    assert isinstance(model, M.DRModelForInference) and model.pooling == "wmean" and model.normalize is True
-    assert loaded["cfg"] == cfg and set(loaded["sd"]) == set(sd)
-    assert all(torch.equal(loaded["sd"][k], sd[k]) for k in sd)       # safetensors round trip is exact (bf16-representable weights)
-
-    # ---- the reference's own encode loop drives the model
-    tok = StubTokenizer(cfg.vocab)
-    pages = synth_doc_pages([(448, 448)] * 7 + [(700, 900), (640, 300), (448, 448)], 31)
-    corpus = [{"id": f"d{i}", "text": "", "image": im} for i, im in enumerate(pages)]
-    queries = [{"id": f"q{i}", "text": t, "image": None} for i, t in enumerate(
-        ["Represent this query for retrieving relevant documents: revenue table", "Represent this query for retrieving relevant documents: climate"])]
-    kw = {"tokenizer": tok, "max_inp_length": 2048}
-    ref_inference(dataset=corpus, model=model, args=enc_args, dataset_type="corpus", split_save=True, model_additional_args=kw)
-    ref_inference(dataset=queries, model=model, args=enc_args, dataset_type="query", split_save=False, model_additional_args=kw)
-    shards = sorted(f for f in os.listdir(out_dir) if f.startswith("embeddings.corpus"))
-    assert shards == ["embeddings.corpus.rank.0.0-6", "embeddings.corpus.rank.0.6-10"]  # flush rule of inference.py:112 at max_inmem_docs=6
-
-    # ---- the reference's retrieve phase over those shards (eval.py:210-232) + metrics through the shim
-    p_ref = O.encode(sd, cfg, tok, [""] * len(pages), pages)
-    q_ref = O.encode(sd, cfg, tok, [q["text"] for q in queries], [None, None])
-    best = np.argmax(q_ref @ p_ref.T, axis=1)
-    qrels_path = str(tmp_path / "qrels.tsv")
-    with open(qrels_path, "w") as f:
-        f.write("query-id\tcorpus-id\tscore\n" + "".join(f"q{i}\td{int(b)}\t1\n" for i, b in enumerate(best)))
-    data_args = SimpleNamespace(from_hf_repo=False, qrels_path=qrels_path)
-    enc_args.phase = "retrieve"
-    ev.retrieve(data_args, enc_args)
-    run = R_load(os.path.join(out_dir, "test.0.trec"))
-    for i, b in enumerate(best):
-        ranked = sorted(run[f"q{i}"].items(), key=lambda kv: -kv[1])
-        assert ranked[0][0] == f"d{int(b)}" and len(ranked) == 4 * len(shards)  # union of per-shard top-5 (dense_retriever.py:88-92)
-    log = open(os.path.join(out_dir, "test_result.log")).read()
-    assert "recall_10" in log or "ndcg_cut_10" in log
-
-
-def R_load(path):
-    from visrag_b200.inference import load_from_trec
-
-    return load_from_trec(path)
+    args.phase = "retrieve"
+    run = R.distributed_parallel_retrieve(args, args.retrieve_depth)
+    I.save_as_trec(run, os.path.join(args.output_dir, "test.0.trec"))
+    ref_path = str(tmp_path / "reference.trec")
+    with open(ref_path, "w") as f:
+        f.write(str(ref["trec_text"]))
+    ref_run = I.load_from_trec(ref_path)
+    got_run = I.load_from_trec(os.path.join(args.output_dir, "test.0.trec"))
+    assert set(got_run) == set(ref_run) == {q["id"] for q in queries}
+    for qid, docs in ref_run.items():
+        got = got_run[qid]
+        assert set(got) == set(docs), qid  # union of per-shard top-4 (dense_retriever.py:88-92)
+        assert max(got, key=got.get) == max(docs, key=docs.get), qid
+        assert max(abs(got[d] - docs[d]) for d in docs) <= 2e-3, qid
